@@ -7,6 +7,7 @@
     python bench.py --model clap-laion-audio --clips 6250          # configs[2]: 50 000 clips over 8 GPUs
     python bench.py --model encodec-emb --clips 1250 --indiv       # configs[3]: 5 000 songs over 4 GPUs, per-song FAD
     python bench.py --model whisper-small --clips 3125 --inf       # configs[4]: 25 000 clips over 8 GPUs, FAD-inf sweep
+    python bench.py --dump-outputs DIR                             # also write the last timed step's results as DIR/*.npy
 
 One "step" = one pass of the whole hot path over the eval set: PCM16 -> front-end -> embedder ->
 fp16 embeddings -> (n, sum, outer-product) statistics -> [all-reduce] -> Frechet distance against
@@ -24,6 +25,11 @@ fixed baseline statistics.  Records of one line:
 `--impl reference` times the reference's CPU implementation of the path (torch-CPU fp32 restatement of the third-party
 model + reference-pinned numpy statistics/Frechet, oracle/) on a bounded sample of the same workload, on every host
 core this process may use (affinity and cgroup quota; torchrun's OMP_NUM_THREADS=1 is overridden).
+`--dump-outputs DIR` (rank 0) writes, after the timing, what the last timed step handed its caller, as float64 .npy:
+  frechet.npy        EvalSetFAD.run_device's fp64[8] (FAD, tr sqrt(C1 C2), residual, iterations, |mu1-mu2|^2, tr C1, tr C2, 0)
+  indiv_scores.npy   with --indiv: every song's FAD, in clip order
+  inf_fit.npy        with --inf: FAD-inf score, slope, r^2
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -374,7 +380,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, default=None,
+                    help="after the timing, write the last timed step's results as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path's results (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     spec = MODELS[args.model]
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -465,6 +477,7 @@ def main():
     ms, _, res = timed(lambda: job.run_device(pcm), args.steps, 0)
     clocks = sampler.stop() if sampler else None
     launches = eng.launches - launches0
+    outputs = {"frechet": res.cpu().numpy()}
     fad_value = float(res[0].item())
     audio_s = total_clips * CLIP_SECONDS * args.steps
     value = audio_s / (ms / 1000.0)
@@ -551,6 +564,7 @@ def main():
                     out = torch.cat(parts)
                 return out.cpu().numpy()                       # the scores the csv is written from
             ms_i, wall_i, scores = timed(indiv_step, args.steps, 1)
+            outputs["indiv_scores"] = scores
             ms_i = max(ms_i, wall_i) / args.steps
             scoring = {"mode": "indiv (score_individual arithmetic: fad_frechet_batched, all songs in lock-step; scores gathered to every rank)",
                        "songs": int(len(scores)), "rows_per_song": rows_per_clip, "d": d,
@@ -582,9 +596,9 @@ def main():
                 slope, intercept = np.polyfit(xs, ys[:, 1], 1)
                 r2 = 1 - np.sum((ys[:, 1] - (slope * xs + intercept)) ** 2) / np.sum((ys[:, 1] - np.mean(ys[:, 1])) ** 2)
                 return intercept, slope, r2
-            n_sw = max(1, args.steps // 2)
-            ms_f, wall_f, (inf_score, inf_slope, inf_r2) = timed(inf_step, n_sw, 1)
-            ms_f = max(ms_f, wall_f) / n_sw
+            ms_f, wall_f, (inf_score, inf_slope, inf_r2) = timed(inf_step, args.steps, 1)
+            outputs["inf_fit"] = np.array([inf_score, inf_slope, inf_r2])
+            ms_f = max(ms_f, wall_f) / args.steps
             scoring = {"mode": "inf (score_inf arithmetic: host RNG indices, gather + exact Gram + Frechet per size on the GPU, sizes sharded over ranks)",
                        "rows": int(n_rows), "d": d, "sizes": 25, "ms_per_sweep": ms_f, "fad_inf": float(inf_score),
                        "slope": float(inf_slope), "r2": float(inf_r2),
@@ -662,6 +676,8 @@ def main():
     if rank != 0:
         dist.shutdown()
         return
+    if args.dump_outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
 
     # ---- CPU baseline + parity sample (rank 0, N = 1 only)
     cpu = None
@@ -688,6 +704,20 @@ def main():
             "cpu_baseline": cpu, "parity_sample": parity}
     print(json.dumps(line))
     dist.shutdown()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(directory: Path, outputs: dict) -> None:
+    """Each array of ``outputs`` as float64 ``directory/<name>.npy``."""
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of results exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    directory.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(directory / f"{name}.npy", a)
 
 
 def files_flow(ml, clips: int, baseline_clips: int, sr: int, workers: int = 16) -> dict:

@@ -94,10 +94,10 @@ def main():
                         cov_with_single_frame_file_is_nan=np.array(bool(np.isnan(cov_n).all())))
     print("stats: mu dtype", mu_c.dtype, "online mu dtype", mu_o.dtype, "nan-case", np.isnan(cov_n).all())
 
-    # 4. FAD-inf (fad.py:304-351) with the global RNG seeded
+    # 4. FAD-inf (fad.py:304-351) with the global RNG seeded; few rows keep the fixture small (about 250 kB)
     rng = np.random.default_rng(77)
-    base = (rng.normal(0, 1, (4000, 128)) * rng.uniform(0.5, 2, 128)).astype(np.float16)
-    evl = (rng.normal(0.1, 1.1, (3000, 128)) * rng.uniform(0.5, 2, 128)).astype(np.float16)
+    base = (rng.normal(0, 1, (256, 128)) * rng.uniform(0.5, 2, 128)).astype(np.float16)
+    evl = (rng.normal(0.1, 1.1, (800, 128)) * rng.uniform(0.5, 2, 128)).astype(np.float16)
     mu_b, cov_b = ref.calc_embd_statistics(base)
     with tempfile.TemporaryDirectory() as tmp:
         np.savez(Path(tmp) / "base.npz", **{"gold.mu": mu_b, "gold.cov": cov_b})

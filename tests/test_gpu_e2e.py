@@ -269,3 +269,23 @@ def test_baseline_config0_sine_vs_noise_one_second_clips(vgg_engine, vgg_state, 
     mu_k, cov_k = fk.calculate_embd_statistics_online(paths["sine"])
     x = cat["sine"].astype(np.float64)
     assert np.abs(mu_k - x.mean(0)).max() < 1e-12 and np.abs(cov_k - np.cov(x, rowvar=False)).max() < 1e-10 * np.abs(cov_k).max()
+
+
+def test_bench_dumps_what_the_last_timed_step_returned(tmp_path):
+    """bench.py --dump-outputs DIR: frechet.npy is the fp64[8] result of the last timed EvalSetFAD.run_device step,
+    the vector the reported FAD is read from."""
+    import json
+    import subprocess
+    import sys
+    from pathlib import Path
+    root = Path(__file__).resolve().parent.parent
+    r = subprocess.run([sys.executable, str(root / "bench.py"), "--clips", "16", "--baseline-clips", "16", "--steps", "2",
+                        "--warmup", "0", "--no-cpu-baseline", "--no-e2e", "--files-clips", "0",
+                        "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=600, cwd=root)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2
+    got = np.load(tmp_path / "out" / "frechet.npy")
+    assert got.dtype == np.float64 and got.shape == (8,)
+    assert got[0] == line["fad"] and np.isfinite(got).all()
+    assert sorted(p.name for p in (tmp_path / "out").iterdir()) == ["frechet.npy"]
